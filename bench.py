@@ -4,6 +4,7 @@
   python bench.py --gpus N --steps K --warmup W                  # this repo's CUDA path, headline = configs[1]
   python bench.py --impl reference --gpus N --steps K ...        # the reference's CPU algorithm on the host cores
   python bench.py --workload composite|pipeline ...              # configs[2] / configs[4] (see below)
+  python bench.py ... --dump-outputs DIR                         # also writes a seeded sample of the last timed step's outputs
 
 Workloads (a step = one pass of the hot path over one batch of synthetic input):
   sort      : configs[1]: 10^8 rows x 64 B (uint64 key + 56-byte payload) per GPU, sort by key.
@@ -32,6 +33,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the (possibly read-only) tree as the build left it
 
 SEED = 0x5954534155525553  # "YTSAURUS" (SURVEY §8d)
 ROW_BYTES = 64
@@ -269,6 +271,23 @@ def verify_sort(out_flat, in_flat, row_bytes, key_cols, world=1, rank=0, dist=No
                     "checksum of whole rows, equal keys keep (source rank, position) order"}
 
 
+def dump_outputs(dirname, outputs, world, rank):
+    """Writes what the last timed step returned, so that two builds can be compared output for output: for every output
+    (name -> (int64 tensor [rows, words], row budget)) a fixed, seeded sample of its rows as <name>.npy, every 64-bit word
+    split into its low and high 32-bit halves (exact in float64), and the sampled row indices as <name>_index.npy.
+    The budgets over all ranks keep the files under 64 MB."""
+    import torch
+    os.makedirs(dirname, exist_ok=True)
+    prefix = f"rank{rank}_" if world > 1 else ""
+    for name, (t, budget) in outputs.items():
+        m = t.shape[0]
+        k = min(m, budget // world)
+        idx = np.sort(np.random.default_rng(SEED).choice(m, k, replace=False))
+        s = t[torch.from_numpy(idx).to(t.device)].cpu().numpy()
+        np.save(os.path.join(dirname, f"{prefix}{name}.npy"), s.view(np.uint32).reshape(k, -1).astype(np.float64))
+        np.save(os.path.join(dirname, f"{prefix}{name}_index.npy"), idx.astype(np.float64))
+
+
 # ------------------------------------------------------------------------------------------------------------
 # GROUP BY (configs[3]) — secondary metric, with its own CPU baselines
 # ------------------------------------------------------------------------------------------------------------
@@ -475,7 +494,10 @@ def main():
                     help="N>1: ytgpu_shuffle_sort (default), the round-1 Python-driven peer scatter, or NCCL all_to_all_single")
     ap.add_argument("--groupby-rows", type=int, default=100_000_000)
     ap.add_argument("--dropin-rows", type=int, default=10_000_000, help="rows of the CreateSortingReader end-to-end leg (C++ adapter)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a seeded sample of the last timed step's outputs to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 0)
     if args.quick:
         args.no_variants = True
@@ -614,6 +636,12 @@ def main():
         parity["checks"]["reduce_keys_increasing"] = bool((gk[1:] > gk[:-1]).all()) if gk.numel() > 1 else True
         parity["ok"] = all(parity["checks"].values())
         del want_s, want_c, got_s, got_c
+    if args.dump_outputs:
+        outputs = {"sorted_rows": (last["out"].view(torch.int64).view(-1, ROW_BYTES // 8), 1 << 18)}
+        if args.workload == "pipeline":
+            g = last["groups"]
+            outputs["groups"] = (torch.stack([reduce_out["keys"][:g], reduce_out["sums"][:g], reduce_out["counts"][:g]], 1), 1 << 17)
+        dump_outputs(args.dump_outputs, outputs, world, rank)
 
     # ---- key-distribution variants of the sort (SURVEY §8d C2) ----
     variants = None

@@ -28,13 +28,14 @@ T_STRING, T_ANY, T_COMPOSITE, T_MAX = 0x10, 0x11, 0x12, 0xEF
 
 
 def build(force: bool = False) -> None:
-    """Compile the oracle (and oracle/_ref when /root/reference is present)."""
+    """Compile the oracle (and oracle/_ref when YTSAURUS_SOURCE_DIR names a YTsaurus source tree)."""
     if force or not os.path.exists(_LIB_PATH) or (
         os.path.getmtime(_LIB_PATH) < os.path.getmtime(os.path.join(_HERE, "yt_oracle.cpp"))
     ):
         subprocess.check_call(["make", "-C", _HERE, "libytoracle.so"])
-    if os.path.isdir("/root/reference") and (force or not os.path.exists(_REF_PATH)):
-        subprocess.check_call(["make", "-C", _HERE, "ref"])
+    src = os.environ.get("YTSAURUS_SOURCE_DIR")
+    if src and os.path.isdir(src) and (force or not os.path.exists(_REF_PATH)):
+        subprocess.check_call(["make", "-C", _HERE, "ref", f"REF={src}"])
 
 
 _lib = None

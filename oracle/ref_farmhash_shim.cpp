@@ -1,5 +1,5 @@
 // Thin extern "C" shim over the REFERENCE's vendored FarmHash, compiled in place from
-// /root/reference/contrib/libs/farmhash/farmhash.cc (never copied into this repo).
+// $YTSAURUS_SOURCE_DIR/contrib/libs/farmhash/farmhash.cc (never copied into this repo).
 // Output: oracle/_ref/libfarmhash_ref.so — used only by tests to validate the oracle's
 // restatement of the fingerprint functions.
 #include <contrib/libs/farmhash/farmhash.h>

@@ -1,5 +1,7 @@
 """Pins the CPU oracle against the reference's own known-answer vectors (tests/golden) and against the
-reference's vendored FarmHash compiled as-is (oracle/_ref).  CPU only."""
+reference's vendored FarmHash (its stored outputs, and its build in oracle/_ref when there is one).  CPU only."""
+import hashlib
+import json
 import os
 import struct
 
@@ -39,20 +41,38 @@ def test_null_and_false_collide():
     assert fps[0] == fps[1] == 0
 
 
-@pytest.mark.skipif(oracle.ref_lib() is None, reason="oracle/_ref not built (no /root/reference)")
+def _seeded(tag, i, n):
+    return hashlib.shake_128(f"{tag} {i}".encode()).digest(n)
+
+
+def _word(tag, i):
+    return int.from_bytes(_seeded(tag, i, 8), "little")
+
+
 def test_farmhash_restatement_matches_reference_build():
+    """The reference's outputs on seeded inputs (tests/golden/farmhash_reference.json), and its build (oracle/_ref)
+    where one was made from a YTsaurus source tree."""
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "farmhash_reference.json")) as f:
+        g = json.load(f)
     ref = oracle.ref_lib()
-    rng = np.random.default_rng(7)
-    for x in [0, 1, 42, 2**63, 2**64 - 1] + [int(v) for v in rng.integers(0, 2**63, 200)]:
-        assert oracle.farm_fingerprint_u64(x) == ref.ref_fingerprint_u64(x)
-    for _ in range(200):
-        lo, hi = (int(v) for v in rng.integers(0, 2**63, 2))
-        assert oracle.farm_fingerprint_u128(lo, hi) == ref.ref_fingerprint_u128(lo, hi)
-        assert oracle.lib().yto_hash128to64(lo, hi) == ref.ref_hash128to64(lo, hi)
+    xs = [0, 1, 42, 2**63, 2**64 - 1] + [_word("u64", i) for i in range(200)]
+    assert len(g["fingerprint_u64"]) == len(xs)
+    for x, want in zip(xs, g["fingerprint_u64"]):
+        assert oracle.farm_fingerprint_u64(x) == int(want), x
+        assert ref is None or ref.ref_fingerprint_u64(x) == int(want), x
+    assert len(g["fingerprint_u128"]) == len(g["hash128to64"]) == 200
+    for i in range(200):
+        lo, hi = _word("u128 lo", i), _word("u128 hi", i)
+        want_fp, want_h = int(g["fingerprint_u128"][i]), int(g["hash128to64"][i])
+        assert oracle.farm_fingerprint_u128(lo, hi) == want_fp and oracle.lib().yto_hash128to64(lo, hi) == want_h, i
+        assert ref is None or (ref.ref_fingerprint_u128(lo, hi) == want_fp and ref.ref_hash128to64(lo, hi) == want_h), i
     # every length class of farmhashna::Hash64: 0, 1-3, 4-7, 8-16, 17-32, 33-64, >64 (incl. multiples of 64)
-    for n in list(range(0, 200)) + [255, 256, 257, 511, 512, 513, 1000, 4096, 65537]:
-        b = rng.integers(0, 256, n, dtype=np.uint8).tobytes()
-        assert oracle.farm_fingerprint_bytes(b) == ref.ref_fingerprint64(b, n), n
+    lengths = list(range(0, 200)) + [255, 256, 257, 511, 512, 513, 1000, 4096, 65537]
+    assert len(g["fingerprint_bytes"]) == len(lengths)
+    for n, want in zip(lengths, g["fingerprint_bytes"]):
+        b = _seeded("bytes", n, n)
+        assert oracle.farm_fingerprint_bytes(b) == int(want), n
+        assert ref is None or ref.ref_fingerprint64(b, n) == int(want), n
 
 
 def test_ordered_partitioner_golden(golden):
