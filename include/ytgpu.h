@@ -62,7 +62,7 @@ uint64_t ytgpu_context_launch_count(const ytgpu_context* ctx);
 /* Device time (ms) of the dominant kernel class measured with CUDA events on the context stream,
  * accumulated since the last reset: which = 0 radix passes that moved data (timed launch by launch), 1 row
  * gather / peer scatter, 2 key extraction, 3 histogram / tie fix-up, 4 partition, 5 group-by, 6 decode / block
- * codec, 7 radix pass launches that were skipped on the device (inactive digit, unarmed fallback), 8 the in-box
+ * codec, 7 radix pass launches that were skipped on the device (inactive digit), 8 the in-box
  * shuffle's row scatter over NVLink, 9 its sampling / pivot selection / count exchange / peer barriers (includes the
  * time spent WAITING for the other ranks), 10 sorted-input segmented reduce.
  * launches (nullable) receives the number of launches behind the returned time. */
@@ -72,7 +72,8 @@ void ytgpu_context_reset_timers(ytgpu_context* ctx);
  * histogram has a single bin are skipped); synchronises the stream. */
 uint64_t ytgpu_context_last_sort_passes(ytgpu_context* ctx);
 void ytgpu_context_enable_timers(ytgpu_context* ctx, int enabled);
-/* Tuning / experiment switches of one context (defaults are the measured-best settings):
+/* Options of one context.  Each chooses between two algorithms that produce the same result; the defaults are the
+ * faster ones.  A new context starts with the defaults:
  *   "sort_hybrid"  1 (default): single-chunk keys are sorted by their most significant active digits first and short
  *                  runs of equal prefixes are fixed up; 0: always the full LSD schedule.
  *   "merge_path"   1 (default): ytgpu_merge_sorted_runs merges up to 16 sorted runs pairwise (merge path); 0: always the

@@ -25,4 +25,4 @@ k = out.view(torch.int64).reshape(n, 8)[:, 0] ^ (-2**63)
 ok = bool((k[1:] >= k[:-1]).all())
 names = ["pass", "gather", "extract", "hist", "part", "groupby", "decode"]
 parts = {names[i]: round(ctx.kernel_ms(i)[0] / steps, 3) for i in range(4)}
-print(f"variant={os.environ.get('YTGPU_SORT_VARIANT','default')} n={n} ms/step={ms:.3f} rows/s={n/ms*1e3:.3e} sorted={ok} {parts} pass_frac={24*n/(parts['pass']/8*1e-3)/1e9/6564.2:.3f}")
+print(f"n={n} ms/step={ms:.3f} rows/s={n/ms*1e3:.3e} sorted={ok} {parts} pass_frac={24*n/(parts['pass']/8*1e-3)/1e9/6564.2:.3f}")

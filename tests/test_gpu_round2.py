@@ -155,6 +155,10 @@ def test_shuffle_entry_points_on_one_rank(ctx):
 
 def test_context_option_sort_hybrid(ctx):
     import torch
+    from ytsaurus_b200 import GpuContext
+    fresh = GpuContext(0)
+    assert fresh.get_option("sort_hybrid") == 1  # a new context reports the default it sorts with
+    fresh.close()
     rng = np.random.default_rng(3)
     n = 300_000
     rows = rng.integers(0, 2**63, (n, 8), dtype=np.int64)
@@ -262,6 +266,13 @@ def test_peer_scatter_validates_caller_supplied_indices(ctx):
     got = torch.cat([d[: int(c) * 64] for d, c in zip(dests, counts)]).cpu().numpy().reshape(-1, 64)
     order = np.argsort(idx, kind="stable")
     assert (got == rows.cpu().numpy().reshape(-1, 64)[order]).all()
+    # more than 32 partitions take the sort-based path
+    idx40 = rng.integers(0, 40, n).astype(np.int32)
+    counts40 = np.bincount(idx40, minlength=40)
+    dests40 = [torch.zeros(n * 64, dtype=torch.uint8, device="cuda") for _ in range(40)]
+    ctx.scatter_rows_to_peers(rows, 64, torch.from_numpy(idx40).cuda(), counts40.tolist(), [d.data_ptr() for d in dests40])
+    got = torch.cat([d[: int(c) * 64] for d, c in zip(dests40, counts40)]).cpu().numpy().reshape(-1, 64)
+    assert (got == rows.cpu().numpy().reshape(-1, 64)[np.argsort(idx40, kind="stable")]).all()
     bad = idx.copy()
     bad[123] = parts + 3
     with pytest.raises(capi.YtGpuError) as e:

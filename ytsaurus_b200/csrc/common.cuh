@@ -77,14 +77,6 @@ __device__ __forceinline__ uint4 ld_stream_u128(const uint4* p) {
                  : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p));
     return v;
 }
-// The same load with the L2 prefetch-size hint set to 64 bytes (SASS: LDG.E.NA.LTC64B): a random 64-byte row then costs
-// one 64-byte DRAM fetch where the default fill brings in the whole 128-byte line.
-__device__ __forceinline__ uint4 ld_stream_u128_l2_64(const uint4* p) {
-    uint4 v;
-    asm volatile("ld.global.nc.L1::no_allocate.L2::64B.v4.u32 {%0,%1,%2,%3}, [%4];"
-                 : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p));
-    return v;
-}
 __device__ __forceinline__ void st_stream_u128(uint4* p, const uint4& v) {
     asm volatile("st.global.L1::no_allocate.v4.u32 [%0], {%1,%2,%3,%4};"
                  :: "l"(p), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w));

@@ -1,7 +1,6 @@
 // context.cu — context lifetime, status plumbing, timers.
 #include <cstdarg>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <new>
 
@@ -101,10 +100,6 @@ int ytgpu_context_create(int device, void* cuda_stream, ytgpu_context** out, ytg
         }
         c->owns_stream = true;
     }
-    if (const char* e = getenv("YTGPU_L2_FETCH")) {
-        // experiment knob: L2 fetch granularity hint (32/64/128 bytes) for the random row/key gathers
-        cudaDeviceSetLimit(cudaLimitMaxL2FetchGranularity, (size_t)atoi(e));
-    }
     // keep freed scratch cached in the stream-ordered pool between calls
     cudaMemPool_t pool;
     if (cudaDeviceGetDefaultMemPool(&pool, device) == cudaSuccess) {
@@ -148,8 +143,8 @@ double ytgpu_context_kernel_ms(ytgpu_context* h, int which, uint64_t* launches) 
     if (which < 0 || which >= KC_COUNT) return 0.0;
     c->collect_timers();
     if (which == KC_RADIX_PASS || which == KC_PASS_SKIPPED) {
-        // Pass launches are timed one by one; launches of skipped digits / the unarmed fallback schedule exit at
-        // once.  A launch counts as "active" when it ran at least a fifth as long as the longest one.
+        // Pass launches are timed one by one; launches of skipped digits exit at once.  A launch counts as "active"
+        // when it ran at least a fifth as long as the longest one.
         float mx = 0;
         for (float f : c->pass_ms) mx = f > mx ? f : mx;
         double act = 0, skip = 0;

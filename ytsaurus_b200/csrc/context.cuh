@@ -33,7 +33,7 @@ struct Context {
     u32 func_attrs_done = 0;
     int opt_merge_path = 1;    // ytgpu_merge_sorted_runs: 1 = merge-path rounds when the runs are few, 0 = always the stable sort
     bool last_merge_used_merge_path = false;
-    int opt_sort_hybrid = -1;  // -1: environment default (YTGPU_SORT_HYBRID, on); 0/1: set through ytgpu_context_set_option
+    int opt_sort_hybrid = 1;   // radix sort: 1 = hybrid MSD-prefix schedule when it applies, 0 = always full LSD
 
     Status alloc(void** p, size_t bytes) {
         if (bytes == 0) bytes = 16;
@@ -144,7 +144,7 @@ struct CtxLock {
 };
 
 // Kernel families whose launches need cudaFuncSetAttribute(MaxDynamicSharedMemorySize) on each device.
-enum FuncAttrFamily : u32 { FA_SORT_PASS = 1u << 0, FA_GATHER_TMA = 1u << 1, FA_GROUPBY = 1u << 2, FA_SHUFFLE = 1u << 3 };
+enum FuncAttrFamily : u32 { FA_SORT_PASS = 1u << 0, FA_GROUPBY = 1u << 2 };
 
 // Reads and clears the device error word (synchronises the stream).
 Status check_device_errors(Context* ctx);

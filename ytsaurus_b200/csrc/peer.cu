@@ -3,7 +3,6 @@
 // reference's "Partition job writes tagged blocks -> Sort job fetches them" hand-off
 // (yt/yt/ytlib/table_client/schemaless_chunk_writer.cpp:1604-1667, partition_chunk_reader.cpp:82-86) is ONE
 // kernel: random 64-byte row reads from local HBM, coalesced row writes over NVLink.  No NCCL call moves rows.
-#include <cstdlib>
 #include <cstring>
 #include <vector>
 
@@ -89,11 +88,10 @@ Status scatter_stream(Context* ctx, const ytgpu_fixed_rows_view* in, const i32* 
     }
     // caller-supplied indices / counts are validated BEFORE anything is written into another GPU's memory
     YTGPU_TRY(check_device_errors(ctx));
-    const char* ord = getenv("YTGPU_SCATTER_ORDERED");
     {
         KernelTimer t(ctx, KC_SCATTER);
         scatter_stream_kernel<<<(u32)tiles, kStreamThreads, 0, ctx->stream>>>(reinterpret_cast<const uint4*>(in->rows), index, n, gr, parts,
-                                                                             bits, tiles, counts.p, D, (ord && ord[0] == '0') ? 0u : 1u);
+                                                                             bits, tiles, counts.p, D);
     }
     YTGPU_CUDA_TRY(cudaGetLastError());
     YTGPU_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
@@ -114,8 +112,7 @@ Status scatter_impl(Context* ctx, const ytgpu_fixed_rows_view* in, const i32* in
     if (start[parts] != n) return make_status(YTGPU_ERR_INVALID_ARGUMENT, "partition row counts sum to %llu, table has %llu rows",
                                               (unsigned long long)start[parts], (unsigned long long)n);
     if (n == 0) return Status{};
-    static const int allow_stream = [] { const char* e = getenv("YTGPU_SCATTER_STREAM"); return e ? atoi(e) : 1; }();
-    if (parts <= kStreamMaxParts && allow_stream) return scatter_stream(ctx, in, index, (u32)parts, start, dest_base);
+    if (parts <= kStreamMaxParts) return scatter_stream(ctx, in, index, (u32)parts, start, dest_base);
     // many partitions: partition index -> sort key chunk -> stable permutation (one radix pass per 256 partitions)
     DevBuf<u64> chunk, dstart;
     DevBuf<void*> ddest;

@@ -117,10 +117,12 @@ struct DestTable {
     u64 start[kStreamMaxParts];    // global slot of its first row (scan value of tile 0)
 };
 
-static __global__ void __launch_bounds__(kStreamThreads) scatter_stream_kernel(const uint4* __restrict__ in, const i32* __restrict__ index,
+// 5 resident CTAs per SM (48 registers): left to itself the compiler takes 54 registers, 4 CTAs per SM, and the 64-byte
+// row scatter measured 12 % slower (1.48 vs 1.32 ms for 5*10^7 rows into 4 partitions; B200 at a 1000 W power limit).
+static __global__ void __launch_bounds__(kStreamThreads, 5) scatter_stream_kernel(const uint4* __restrict__ in, const i32* __restrict__ index,
                                                                         u64 n, u32 gr, u32 parts, u32 part_bits, u64 tiles,
                                                                         const u64* __restrict__ tile_base /*[parts][tiles]*/,
-                                                                        const DestTable D, u32 ordered) {
+                                                                        const DestTable D) {
     constexpr int WARPS = kStreamThreads / 32;
     __shared__ u32 s_wcnt[WARPS][kStreamMaxParts];  // running per-warp counts -> warp offsets inside the tile
     __shared__ u64 s_slot[kStreamMaxParts];         // first slot of this tile per partition
@@ -194,7 +196,7 @@ static __global__ void __launch_bounds__(kStreamThreads) scatter_stream_kernel(c
             // Rows leave in destination order: rows of one partition sit next to each other in its slab, so a store
             // instruction writes runs of whole rows (128 B and more) instead of isolated 64-byte rows — fewer, larger
             // NVLink write packets.
-            s_order[warp][ordered ? pos[i] : lane] = (u8)lane;
+            s_order[warp][pos[i]] = (u8)lane;
             __syncwarp();
 #pragma unroll
             for (u32 s = 0; s < 4; ++s) {
@@ -218,99 +220,6 @@ static __global__ void __launch_bounds__(kStreamThreads) scatter_stream_kernel(c
         for (u32 g = 0; g < gr; ++g) dst[g] = ld_stream_u128(src + g);
     }
     __threadfence_system();
-}
-
-
-// ---------------------------------------------------------------------------------------------
-// Tile-staged scatter for 64-byte rows: the whole 1024-row tile is staged in shared memory IN DESTINATION ORDER, then
-// written out with consecutive threads -> consecutive 16-byte granules.  A store instruction then covers 512 contiguous
-// bytes of ONE destination slab (the per-warp variant above writes runs of ~32/g rows: 256 B at g = 8), i.e. fewer and
-// larger NVLink write packets: what limits the exchange at 4-8 GPUs.
-// ---------------------------------------------------------------------------------------------
-constexpr size_t kScatterTileSmem = (size_t)kStreamTile * 64;
-
-static __global__ void __launch_bounds__(kStreamThreads) scatter_tile_kernel(const uint4* __restrict__ in, const i32* __restrict__ index, u64 n,
-                                                                             u32 parts, u32 part_bits, u64 tiles,
-                                                                             const u64* __restrict__ tile_base /*[parts][tiles]*/, const DestTable D) {
-    constexpr int WARPS = kStreamThreads / 32;
-    extern __shared__ __align__(16) uint4 s_tile[];         // [kStreamTile][4]
-    __shared__ u32 s_wcnt[WARPS][kStreamMaxParts];           // per-warp counts -> warp offsets inside the partition's tile segment
-    __shared__ u32 s_pstart[kStreamMaxParts + 1];            // first tile slot of every partition
-    __shared__ uint4* s_gptr[kStreamMaxParts];               // where this tile's rows of partition p start in p's destination slab
-    __shared__ u8 s_dest[kStreamTile];                       // partition of every tile slot
-    const u32 tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    if (tid < WARPS * kStreamMaxParts) (&s_wcnt[0][0])[tid] = 0;
-    __syncthreads();
-    const u64 tile = blockIdx.x;
-    const u64 wbase = tile * kStreamTile + (u64)warp * (32 * kStreamItems) + lane;  // warp-striped: stable (item, lane) order
-    u32 part[kStreamItems], rank[kStreamItems];
-    u32 lt;
-    asm("mov.u32 %0, %%lanemask_lt;" : "=r"(lt));
-#pragma unroll
-    for (int i = 0; i < kStreamItems; ++i) {
-        const u64 r = wbase + (u64)i * 32;
-        const bool valid = r < n;
-        part[i] = valid ? min((u32)index[r], parts - 1) : 0u;
-        const u32 kk = valid ? part[i] : (1u << part_bits);
-        u32 m = 0xffffffffu;
-        for (int b = (int)part_bits; b >= 0; --b) {
-            const bool bit = (kk >> b) & 1;
-            const u32 v = __ballot_sync(0xffffffffu, bit);
-            m &= bit ? v : ~v;
-        }
-        const u32 prev = s_wcnt[warp][part[i]];
-        __syncwarp();
-        if (valid && (m & lt) == 0) s_wcnt[warp][part[i]] = prev + __popc(m);
-        rank[i] = prev + __popc(m & lt);
-        __syncwarp();
-    }
-    __syncthreads();
-    if (tid < parts) {
-        u32 run = 0;
-#pragma unroll
-        for (int w = 0; w < WARPS; ++w) {
-            const u32 c = s_wcnt[w][tid];
-            s_wcnt[w][tid] = run;
-            run += c;
-        }
-        s_pstart[tid + 1] = run;  // counts for now
-        s_gptr[tid] = D.base[tid] + (tile_base[(u64)tid * tiles + tile] - D.start[tid]) * 4;
-    }
-    __syncthreads();
-    if (tid == 0) {
-        u32 run = 0;
-        s_pstart[0] = 0;
-        for (u32 p = 0; p < parts; ++p) {
-            const u32 c = s_pstart[p + 1];
-            s_pstart[p + 1] = run + c;
-            run += c;
-        }
-    }
-    __syncthreads();
-    // stage: the 32 rows of a round are contiguous in the input (one coalesced 2 KB read); row `row` of the round goes to
-    // the tile slot its owner lane computed
-#pragma unroll
-    for (int i = 0; i < kStreamItems; ++i) {
-        const u64 r = wbase + (u64)i * 32;
-        const u32 p = part[i];
-        const u32 myslot = r < n ? s_pstart[p] + s_wcnt[warp][p] + rank[i] : 0xffffffffu;
-        if (r < n) s_dest[myslot] = (u8)p;
-        const u64 round_row0 = r - lane;
-#pragma unroll
-        for (u32 s4 = 0; s4 < 4; ++s4) {
-            const u32 q = s4 * 32 + lane, row = q >> 2, g = q & 3;
-            const u32 slot = __shfl_sync(0xffffffffu, myslot, row);
-            if (slot != 0xffffffffu) s_tile[slot * 4 + g] = ld_stream_u128(in + round_row0 * 4 + q);
-        }
-    }
-    __syncthreads();
-    const u32 total = s_pstart[parts] * 4;  // granules
-    for (u32 q = tid; q < total; q += kStreamThreads) {
-        const u32 slot = q >> 2, g = q & 3;
-        const u32 p = s_dest[slot];
-        s_gptr[p][(size_t)(slot - s_pstart[p]) * 4 + g] = s_tile[q];
-    }
-    __threadfence_system();  // peer stores are ordered before whatever signals completion to the other GPU
 }
 
 }  // namespace ytgpu

@@ -5,7 +5,6 @@
 //   10k-bucket std::sort + heap merge yt/yt/ytlib/table_client/partition_sort_reader.cpp:461-529
 // with a stable radix sort over order-preserving normalised keys (keys.cuh).
 #include <algorithm>
-#include <cstdlib>
 #include <vector>
 
 #include "radix_sort.cuh"
@@ -332,7 +331,7 @@ struct PassParams {
     u32* counter;           // dynamic tile id, zeroed
     const SortPlan* plan;
     int plan_index;
-    int schedule;  // 0: plan->pass[plan_index]; 1: plan->pass_b[plan_index], runs only when plan->fallback
+    int schedule;  // 0: plan->pass[plan_index]; 1: plan->pass_b[plan_index], launched only after plan->fallback is set
     int shift;
     u32 n;
 };
@@ -531,29 +530,21 @@ __global__ void __launch_bounds__(THREADS, MINB) onesweep_pass_kernel(const Pass
     u32* s_hist = reinterpret_cast<u32*>(smem_raw + (size_t)TILE * 12);
     u32* s_misc = s_hist + WARPS * kRadix + 2 * kRadix;
 
-    if (P.schedule == 1 && !P.plan->fallback) return;
     const PassDesc pd = P.schedule == 1 ? P.plan->pass_b[P.plan_index] : P.plan->pass[P.plan_index];
     if (!pd.active) return;
     // One tile per CTA.  (A persistent variant — 3 CTAs per SM looping over an atomic tile counter — measured 8 %
     // slower on the active passes: 6.51 vs 5.96 ms for 8 passes over 10^8 rows; hardware CTA launch is cheaper
     // than the extra barrier per tile.)  Tile ids still come from the atomic counter so that they are handed
     // out in start order, which the decoupled look-back relies on.
-    // The rarely armed fallback schedule is launched with a small persistent grid (gridDim < tiles) so that its
-    // eight normally idle launches cost a few microseconds instead of `tiles` empty CTAs each.
     const u32 tiles = (u32)(((u64)P.n + TILE - 1) / TILE);
-    const bool persistent = gridDim.x < tiles;
-    for (;;) {
-        if (threadIdx.x == 0) s_misc[8] = atomicAdd(P.counter, 1u);
+    if (threadIdx.x == 0) s_misc[8] = atomicAdd(P.counter, 1u);
 #pragma unroll
-        for (int i = threadIdx.x; i < WARPS * kRadix; i += THREADS) s_hist[i] = 0;
-        __syncthreads();
-        const u32 tile = s_misc[8];
-        if (tile >= tiles) break;
-        if ((u64)(tile + 1) * TILE <= (u64)P.n) onesweep_tile<THREADS, ITEMS, true>(P, pd, tile, smem_raw);
-        else onesweep_tile<THREADS, ITEMS, false>(P, pd, tile, smem_raw);
-        if (!persistent) break;
-        __syncthreads();  // everyone is done with this tile's shared memory
-    }
+    for (int i = threadIdx.x; i < WARPS * kRadix; i += THREADS) s_hist[i] = 0;
+    __syncthreads();
+    const u32 tile = s_misc[8];
+    if (tile >= tiles) return;
+    if ((u64)(tile + 1) * TILE <= (u64)P.n) onesweep_tile<THREADS, ITEMS, true>(P, pd, tile, smem_raw);
+    else onesweep_tile<THREADS, ITEMS, false>(P, pd, tile, smem_raw);
 }
 
 __global__ void materialize_perm_kernel(const SortPlan* plan, const u32* a, const u32* b, u64 n, u32* dst) {
@@ -565,35 +556,27 @@ constexpr size_t pass_smem_bytes(int items) {
     return (size_t)kSortThreads * items * 12 + (size_t)(kSortThreads / 32) * kRadix * 4 + 2 * kRadix * 4 + 16 * 4;
 }
 
-// Tuning variants of the pass kernel (items per thread, min resident CTAs per SM); YTGPU_SORT_VARIANT
-// selects one for experiments, the default is the best measured on B200 (profiles/).
-struct PassVariant {
-    int items;
-    int ctas_per_sm;
-    void (*kernel)(const PassParams);
-};
-const PassVariant kVariants[] = {
-    {16, 2, onesweep_pass_kernel<kSortThreads, 16, 2>},
-    {16, 3, onesweep_pass_kernel<kSortThreads, 16, 3>},
-    {12, 3, onesweep_pass_kernel<kSortThreads, 12, 3>},
-    {8, 4, onesweep_pass_kernel<kSortThreads, 8, 4>},
-    {12, 4, onesweep_pass_kernel<kSortThreads, 12, 4>},
-    {20, 2, onesweep_pass_kernel<kSortThreads, 20, 2>},
-};
-constexpr int kDefaultVariant = 1;
+// 16 items per thread at 3 resident CTAs per SM measured best on B200 (DESIGN.md §4).
+constexpr int kSortItems = 16;
+constexpr int kSortCtasPerSm = 3;
 
-const PassVariant& pass_variant(Context* ctx) {
-    static const int v = [] {
-        const char* e = getenv("YTGPU_SORT_VARIANT");
-        int x = e ? atoi(e) : kDefaultVariant;
-        if (x < 0 || x >= (int)(sizeof(kVariants) / sizeof(kVariants[0]))) x = kDefaultVariant;
-        return x;
-    }();
+void prepare_pass_kernel(Context* ctx) {
     if (!(ctx->func_attrs_done & FA_SORT_PASS)) {  // per device (the attribute belongs to the current device's function)
-        cudaFuncSetAttribute(kVariants[v].kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pass_smem_bytes(kVariants[v].items));
+        cudaFuncSetAttribute(onesweep_pass_kernel<kSortThreads, kSortItems, kSortCtasPerSm>,
+                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pass_smem_bytes(kSortItems));
         ctx->func_attrs_done |= FA_SORT_PASS;
     }
-    return kVariants[v];
+}
+
+// Allocates and fills s->hist with the raw digit counts of every chunk.
+Status histogram_chunks(Context* ctx, const u64* const* chunks, int nchunks, u64 n, SortScratch* s) {
+    YTGPU_TRY(prepare_histogram(ctx, nchunks, s));
+    KernelTimer t(ctx, KC_HISTOGRAM, nchunks);
+    const u64 per_block = (u64)kHistThreads * kHistItems;
+    const u32 blocks = (u32)std::min<u64>((n + per_block - 1) / per_block, (u64)kNumSms * 4);
+    for (int c = 0; c < nchunks; ++c)
+        histogram_kernel<<<blocks, kHistThreads, 0, ctx->stream>>>(chunks[c], n, s->hist.p + (size_t)c * kPassesPerChunk * kRadix);
+    return Status{};
 }
 
 }  // namespace
@@ -652,55 +635,47 @@ Status radix_sort_chunks(Context* ctx, const u64* const* chunks, int nchunks, u6
                            (unsigned long long)n);
     cudaStream_t st = ctx->stream;
     YTGPU_CUDA_TRY(cudaSetDevice(ctx->device));
-    const PassVariant& pv = pass_variant(ctx);
-    const u32 tile_rows = (u32)kSortThreads * pv.items;
+    prepare_pass_kernel(ctx);
+    const u32 tile_rows = (u32)kSortThreads * kSortItems;
     const u32 tiles = (u32)((n + tile_rows - 1) / tile_rows);
     const int total_passes = nchunks * kPassesPerChunk;
-    const u32 grid = tiles;
 
     YTGPU_TRY(s->keys[0].allocate(ctx, n));
     YTGPU_TRY(s->keys[1].allocate(ctx, n));
     YTGPU_TRY(s->idx[0].allocate(ctx, n));
     YTGPU_TRY(s->idx[1].allocate(ctx, n));
-    if (!s->hist_precomputed) YTGPU_TRY(prepare_histogram(ctx, nchunks, s));
+    if (!s->hist_precomputed) YTGPU_TRY(histogram_chunks(ctx, chunks, nchunks, n, s));
     YTGPU_TRY(s->status.allocate(ctx, (size_t)kPassesPerChunk * tiles * kRadix));
     YTGPU_TRY(s->counters.allocate(ctx, (size_t)total_passes + kPassesPerChunk));
     YTGPU_TRY(s->plan.allocate(ctx, 1));
 
     YTGPU_CUDA_TRY(cudaMemsetAsync(s->counters.p, 0, ((size_t)total_passes + kPassesPerChunk) * 4, st));
-    static const int env_hybrid = [] { const char* e = getenv("YTGPU_SORT_HYBRID"); return e ? atoi(e) : 1; }();
-    const int allow_hybrid = (ctx->opt_sort_hybrid >= 0 ? ctx->opt_sort_hybrid : env_hybrid) && !s->no_hybrid && n >= kHybridMinRows;
-
-    if (!s->hist_precomputed) {
-        KernelTimer t(ctx, KC_HISTOGRAM, nchunks);
-        u64 per_block = (u64)kHistThreads * kHistItems;
-        u32 blocks = (u32)std::min<u64>((n + per_block - 1) / per_block, (u64)kNumSms * 4);
-        for (int c = 0; c < nchunks; ++c)
-            histogram_kernel<<<blocks, kHistThreads, 0, st>>>(chunks[c], n, s->hist.p + (size_t)c * kPassesPerChunk * kRadix);
-    }
+    const int allow_hybrid = ctx->opt_sort_hybrid && !s->no_hybrid && n >= kHybridMinRows;
     plan_kernel<<<1, 256, 0, st>>>(s->hist.p, nchunks, (u32)n, s->plan.p, allow_hybrid, s->keep_keys ? 1 : 0);
     ctx->count_launch();
 
+    // Digit p of chunk r, from the plan's main schedule (0) or its complete fallback schedule (1, single chunk only).
+    auto launch_pass = [&](int r, int p, int schedule) {
+        KernelTimer t(ctx, KC_RADIX_PASS);
+        PassParams P;
+        P.chunk = chunks[r];
+        P.keys[0] = s->keys[0].p;
+        P.keys[1] = s->keys[1].p;
+        P.idx[0] = s->idx[0].p;
+        P.idx[1] = s->idx[1].p;
+        P.digit_base = s->hist.p + (size_t)(r * kPassesPerChunk + p) * kRadix;
+        P.status = s->status.p + (size_t)p * tiles * kRadix;
+        P.counter = s->counters.p + (schedule * total_passes + r * kPassesPerChunk + p);
+        P.plan = s->plan.p;
+        P.plan_index = r * kPassesPerChunk + p;
+        P.schedule = schedule;
+        P.shift = p * kRadixBits;
+        P.n = (u32)n;
+        onesweep_pass_kernel<kSortThreads, kSortItems, kSortCtasPerSm><<<tiles, kSortThreads, pass_smem_bytes(kSortItems), st>>>(P);
+    };
     for (int r = nchunks - 1; r >= 0; --r) {
         YTGPU_CUDA_TRY(cudaMemsetAsync(s->status.p, 0, (size_t)kPassesPerChunk * tiles * kRadix * 4, st));
-        for (int p = 0; p < kPassesPerChunk; ++p) {
-            KernelTimer t(ctx, KC_RADIX_PASS);
-            PassParams P;
-            P.chunk = chunks[r];
-            P.keys[0] = s->keys[0].p;
-            P.keys[1] = s->keys[1].p;
-            P.idx[0] = s->idx[0].p;
-            P.idx[1] = s->idx[1].p;
-            P.digit_base = s->hist.p + (size_t)(r * kPassesPerChunk + p) * kRadix;
-            P.status = s->status.p + (size_t)p * tiles * kRadix;
-            P.counter = s->counters.p + (r * kPassesPerChunk + p);
-            P.plan = s->plan.p;
-            P.plan_index = r * kPassesPerChunk + p;
-            P.schedule = 0;
-            P.shift = p * kRadixBits;
-            P.n = (u32)n;
-            pv.kernel<<<grid, kSortThreads, pass_smem_bytes(pv.items), st>>>(P);
-        }
+        for (int p = 0; p < kPassesPerChunk; ++p) launch_pass(r, p, 0);
     }
     if (nchunks == 1 && allow_hybrid) {
         // hybrid tail: order the short runs of equal prefixes, classify the long ones
@@ -731,24 +706,7 @@ Status radix_sort_chunks(Context* ctx, const u64* const* chunks, int nchunks, u6
                 const u32 one = 1;
                 YTGPU_CUDA_TRY(cudaMemcpyAsync(&s->plan.p->fallback, &one, 4, cudaMemcpyHostToDevice, st));
                 YTGPU_CUDA_TRY(cudaMemsetAsync(s->status.p, 0, (size_t)kPassesPerChunk * tiles * kRadix * 4, st));
-                for (int p = 0; p < kPassesPerChunk; ++p) {
-                    KernelTimer t(ctx, KC_RADIX_PASS);
-                    PassParams P;
-                    P.chunk = chunks[0];
-                    P.keys[0] = s->keys[0].p;
-                    P.keys[1] = s->keys[1].p;
-                    P.idx[0] = s->idx[0].p;
-                    P.idx[1] = s->idx[1].p;
-                    P.digit_base = s->hist.p + (size_t)p * kRadix;
-                    P.status = s->status.p + (size_t)p * tiles * kRadix;
-                    P.counter = s->counters.p + (total_passes + p);
-                    P.plan = s->plan.p;
-                    P.plan_index = p;
-                    P.schedule = 1;
-                    P.shift = p * kRadixBits;
-                    P.n = (u32)n;
-                    pv.kernel<<<grid, kSortThreads, pass_smem_bytes(pv.items), st>>>(P);
-                }
+                for (int p = 0; p < kPassesPerChunk; ++p) launch_pass(0, p, 1);
                 YTGPU_CUDA_TRY(cudaStreamSynchronize(st));  // `one` lives on this stack frame
             } else {
                 YTGPU_TRY(sort_mixed_runs(ctx, s, hs, mixedlist.p));
@@ -909,8 +867,7 @@ __global__ void __launch_bounds__(256) deep_tie_fix_kernel(const SortPlan* plan,
 }  // namespace
 
 Status radix_sort_keys(Context* ctx, const u64* const* chunks, int nchunks, u64 n, SortScratch* s, PermRef* out) {
-    static const int env_prefix = [] { const char* e = getenv("YTGPU_SORT_PREFIX_CHUNK"); return e ? atoi(e) : 1; }();
-    if (nchunks == 1 || n < 2 || !env_prefix) return radix_sort_chunks(ctx, chunks, nchunks, n, s, out);
+    if (nchunks == 1 || n < 2) return radix_sort_chunks(ctx, chunks, nchunks, n, s, out);
     if (nchunks < 1 || nchunks > kMaxKeyChunks)
         return make_status(YTGPU_ERR_UNSUPPORTED, "normalised key of %d bytes exceeds the %d-byte limit", nchunks * 8, kMaxKeyChunks * 8);
     if (n >= (1ull << 30))
@@ -919,12 +876,7 @@ Status radix_sort_keys(Context* ctx, const u64* const* chunks, int nchunks, u64 
     YTGPU_CUDA_TRY(cudaSetDevice(ctx->device));
     // 1. raw digit counts of every chunk (the complete schedule needs them as well)
     if (!s->hist_precomputed) {
-        YTGPU_TRY(prepare_histogram(ctx, nchunks, s));
-        KernelTimer t(ctx, KC_HISTOGRAM, nchunks);
-        const u64 per_block = (u64)kHistThreads * kHistItems;
-        const u32 blocks = (u32)std::min<u64>((n + per_block - 1) / per_block, (u64)kNumSms * 4);
-        for (int c = 0; c < nchunks; ++c)
-            histogram_kernel<<<blocks, kHistThreads, 0, st>>>(chunks[c], n, s->hist.p + (size_t)c * kPassesPerChunk * kRadix);
+        YTGPU_TRY(histogram_chunks(ctx, chunks, nchunks, n, s));
         s->hist_precomputed = true;
     }
     // 2. prefix chunk of the 8 most significant active bytes + its histogram

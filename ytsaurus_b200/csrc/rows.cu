@@ -3,8 +3,6 @@
 // The gather replaces TSortingReader::Read serving rows in sorted order
 // (yt/yt/ytlib/table_client/sorting_reader.cpp:58-81) and TPartitionSortReader::Read's
 // JumpToRowIndex + GetRow random-access decode (partition_sort_reader.cpp:136-146).
-#include <cstdlib>
-
 #include "rows.cuh"
 
 namespace ytgpu {
@@ -185,8 +183,8 @@ __global__ void __launch_bounds__(256) max_string_length_kernel(const WidthCols 
 }
 
 // ---- gather: 16-byte granules; GR granules per row; each thread moves UNROLL granules ----
-// STREAM: 0 = default loads / stores, 1 = L1::no_allocate, 2 = L1::no_allocate + L2::64B prefetch size on the row reads
-template <int UNROLL, bool PLAIN, int STREAM = 1>
+// Loads and stores bypass L1 (L1::no_allocate): every granule is touched once.
+template <int UNROLL, bool PLAIN>
 __global__ void __launch_bounds__(256) gather_rows_kernel(const uint4* __restrict__ in, const SortPlan* plan,
                                                           const u32* __restrict__ pa, const u32* __restrict__ pb,
                                                           uint4* __restrict__ out, u64 n, u32 gr, u32 gr_shift) {
@@ -213,104 +211,15 @@ __global__ void __launch_bounds__(256) gather_rows_kernel(const uint4* __restric
                     g = (u32)(q - j * gr);
                 }
                 u64 src = (f == 2 ? j : (u64)perm[j]);
-                v[k] = STREAM == 2 ? ld_stream_u128_l2_64(in + src * gr + g) : (STREAM ? ld_stream_u128(in + src * gr + g) : in[src * gr + g]);
+                v[k] = ld_stream_u128(in + src * gr + g);
             }
         }
 #pragma unroll
         for (int k = 0; k < UNROLL; ++k) {
             u64 q = q0 + (u64)k * stride;
-            if (ok[k]) {
-                if (STREAM) st_stream_u128(out + q, v[k]);
-                else out[q] = v[k];
-            }
+            if (ok[k]) st_stream_u128(out + q, v[k]);
         }
     }
-}
-
-// ---- TMA gather: rows are staged through shared memory with 1-D bulk copies ----
-// Each CTA loops over tiles of TMA_ROWS rows: every thread issues cp.async.bulk (global -> shared,
-// row_bytes each, completion counted on an mbarrier) for its rows, then one thread stores the whole
-// contiguous tile with a single bulk shared -> global copy.  STAGES tiles are in flight per CTA.
-__device__ __forceinline__ u32 smem_u32(const void* p) { return (u32)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(u64* bar, u32 count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(u64* bar, u32 bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(u64* bar, u32 parity) {
-    u32 done = 0;
-    while (!done) {
-        asm volatile(
-            "{\n"
-            ".reg .pred p;\n"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n"
-            "selp.u32 %0, 1, 0, p;\n"
-            "}\n" : "=r"(done) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-    }
-}
-__device__ __forceinline__ void bulk_g2s(void* dst_smem, const void* src_gmem, u32 bytes, u64* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 :: "r"(smem_u32(dst_smem)), "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void bulk_s2g(void* dst_gmem, const void* src_smem, u32 bytes) {
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;"
-                 :: "l"(dst_gmem), "r"(smem_u32(src_smem)), "r"(bytes) : "memory");
-}
-
-constexpr int kTmaThreads = 128;
-constexpr int kTmaStages = 4;
-
-template <bool PLAIN>
-__global__ void __launch_bounds__(kTmaThreads) gather_rows_tma_kernel(const u8* __restrict__ in, const SortPlan* plan,
-                                                                      const u32* __restrict__ pa, const u32* __restrict__ pb,
-                                                                      u8* __restrict__ out, u64 n, u32 row_bytes, u32 tile_rows) {
-    extern __shared__ __align__(128) unsigned char tma_smem[];
-    __shared__ __align__(8) u64 bars[kTmaStages];
-    const u32 f = PLAIN ? 0u : plan_final_idx(plan);
-    const u32* perm = f == 1 ? pb : pa;
-    const u32 tile_bytes = tile_rows * row_bytes;
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < kTmaStages; ++s) mbar_init(&bars[s], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    const u64 tiles = (n + tile_rows - 1) / tile_rows;
-    u32 it = 0;
-    u64 prev_row0 = 0;
-    u32 prev_rows = 0;
-    for (u64 tile = blockIdx.x; tile < tiles; tile += gridDim.x, ++it) {
-        const u32 stage = it % kTmaStages;
-        unsigned char* buf = tma_smem + (size_t)stage * tile_bytes;
-        const u64 row0 = tile * tile_rows;
-        const u32 rows_here = (u32)min((u64)tile_rows, n - row0);
-        if (threadIdx.x == 0) {
-            // the bulk store that used this stage kTmaStages tiles ago must be done reading it
-            asm volatile("cp.async.bulk.wait_group.read %0;" :: "n"(kTmaStages - 2) : "memory");
-            mbar_expect_tx(&bars[stage], rows_here * row_bytes);
-        }
-        __syncthreads();
-        for (u32 r = threadIdx.x; r < rows_here; r += kTmaThreads) {
-            const u64 j = row0 + r;
-            const u64 src = f == 2 ? j : (u64)perm[j];
-            bulk_g2s(buf + (size_t)r * row_bytes, in + src * row_bytes, row_bytes, &bars[stage]);
-        }
-        if (threadIdx.x == 0 && it > 0) {  // previous tile: wait for its rows, store it in one piece
-            const u32 ps = (it - 1) % kTmaStages;
-            mbar_wait(&bars[ps], ((it - 1) / kTmaStages) & 1);
-            bulk_s2g(out + prev_row0 * row_bytes, tma_smem + (size_t)ps * tile_bytes, prev_rows * row_bytes);
-            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-        }
-        prev_row0 = row0;
-        prev_rows = rows_here;
-    }
-    if (threadIdx.x == 0 && it > 0) {
-        const u32 ps = (it - 1) % kTmaStages;
-        mbar_wait(&bars[ps], ((it - 1) / kTmaStages) & 1);
-        bulk_s2g(out + prev_row0 * row_bytes, tma_smem + (size_t)ps * tile_bytes, prev_rows * row_bytes);
-        asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-    }
-    if (threadIdx.x == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
 }
 
 __global__ void __launch_bounds__(256) widen_index_kernel(const i32* __restrict__ in, u64 n, u64* __restrict__ out) {
@@ -396,42 +305,12 @@ static Status gather_launch(Context* ctx, const u8* in_dev, const SortPlan* plan
     u32 gr = row_bytes / 16;
     u32 shift = (gr & (gr - 1)) == 0 ? (u32)__builtin_ctz(gr) : 0xffffffffu;
     KernelTimer t(ctx, KC_GATHER);
-    static const int variant = [] { const char* e = getenv("YTGPU_GATHER_VARIANT"); return e ? atoi(e) : 0; }();
-    if (variant >= 2) {
-        // TMA bulk-copy staging; tile rows chosen so that kTmaStages tiles fit comfortably
-        const u32 tile_rows = variant == 2 ? 128 : 256;
-        const size_t smem = (size_t)kTmaStages * tile_rows * row_bytes;
-        if (smem <= 200 * 1024) {
-            if (!(ctx->func_attrs_done & FA_GATHER_TMA)) {
-                cudaFuncSetAttribute(gather_rows_tma_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-                cudaFuncSetAttribute(gather_rows_tma_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-                ctx->func_attrs_done |= FA_GATHER_TMA;
-            }
-            const u64 tiles = (n + tile_rows - 1) / tile_rows;
-            const u32 per_sm = (u32)std::max<size_t>(1, std::min<size_t>(8, (220 * 1024) / (smem + 1024)));
-            const u32 grid = (u32)std::min<u64>(tiles, (u64)kNumSms * per_sm);
-            if (plain)
-                gather_rows_tma_kernel<true><<<grid, kTmaThreads, smem, ctx->stream>>>(in_dev, nullptr, pa, pb, out_dev, n, row_bytes, tile_rows);
-            else
-                gather_rows_tma_kernel<false><<<grid, kTmaThreads, smem, ctx->stream>>>(in_dev, plan, pa, pb, out_dev, n, row_bytes, tile_rows);
-            YTGPU_CUDA_TRY(cudaGetLastError());
-            return Status{};
-        }
-    }
     constexpr int UNROLL = 4;
     u32 grid = grid_for((n * gr + UNROLL - 1) / UNROLL, 256, 8);
     const uint4* in4 = reinterpret_cast<const uint4*>(in_dev);
     uint4* out4 = reinterpret_cast<uint4*>(out_dev);
-    if (variant == 1) {
-        if (plain) gather_rows_kernel<UNROLL, true, 0><<<grid, 256, 0, ctx->stream>>>(in4, nullptr, pa, pb, out4, n, gr, shift);
-        else gather_rows_kernel<UNROLL, false, 0><<<grid, 256, 0, ctx->stream>>>(in4, plan, pa, pb, out4, n, gr, shift);
-    } else if (variant == -1 && row_bytes <= 64) {  // experiment: 64-byte L2 fills for rows that do not fill a 128-byte line
-        if (plain) gather_rows_kernel<UNROLL, true, 2><<<grid, 256, 0, ctx->stream>>>(in4, nullptr, pa, pb, out4, n, gr, shift);
-        else gather_rows_kernel<UNROLL, false, 2><<<grid, 256, 0, ctx->stream>>>(in4, plan, pa, pb, out4, n, gr, shift);
-    } else {
-        if (plain) gather_rows_kernel<UNROLL, true><<<grid, 256, 0, ctx->stream>>>(in4, nullptr, pa, pb, out4, n, gr, shift);
-        else gather_rows_kernel<UNROLL, false><<<grid, 256, 0, ctx->stream>>>(in4, plan, pa, pb, out4, n, gr, shift);
-    }
+    if (plain) gather_rows_kernel<UNROLL, true><<<grid, 256, 0, ctx->stream>>>(in4, nullptr, pa, pb, out4, n, gr, shift);
+    else gather_rows_kernel<UNROLL, false><<<grid, 256, 0, ctx->stream>>>(in4, plan, pa, pb, out4, n, gr, shift);
     YTGPU_CUDA_TRY(cudaGetLastError());
     return Status{};
 }

@@ -17,7 +17,6 @@
 //                   buffer over NVLink (peer_kernels.cuh), barrier
 //   local sort   -> the rank's key range (capi_sort.cu)
 // The host takes part once per sort (it reads the count matrix to size the local sort); no NCCL, no host barrier.
-#include <cstdlib>
 #include <cstring>
 #include <new>
 #include <vector>
@@ -407,21 +406,11 @@ Status shuffle_sort_impl(Shuffle* s, const ytgpu_fixed_rows_view* in, const ytgp
         u32 bits = 0;
         while ((1u << bits) < parts) ++bits;
         KernelTimer t(ctx, KC_SCATTER);
-        // The tile-staged scatter (rows regrouped by destination in shared memory first) is opt-in: measured at 2 ranks it
-        // is SLOWER than the streaming one (6.64 vs 4.97 ms for 5*10^7 rows out: the streaming kernel's 64-byte row
-        // stores already fill whole NVLink packets, staging only adds a shared-memory round trip and a barrier).
-        static const int tile_scatter = [] { const char* e = getenv("YTGPU_SCATTER_TILE"); return e ? atoi(e) : 0; }();
-        if (rb == 64 && tile_scatter) {
-            if (!(ctx->func_attrs_done & FA_SHUFFLE)) {
-                cudaFuncSetAttribute(scatter_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kScatterTileSmem);
-                ctx->func_attrs_done |= FA_SHUFFLE;
-            }
-            scatter_tile_kernel<<<(u32)tiles, kStreamThreads, kScatterTileSmem, st>>>(reinterpret_cast<const uint4*>(in->rows), index.p, n, parts, bits,
-                                                                                      tiles, counts.p, D);
-        } else {
-            scatter_stream_kernel<<<(u32)tiles, kStreamThreads, 0, st>>>(reinterpret_cast<const uint4*>(in->rows), index.p, n, rb / 16, parts, bits,
-                                                                        tiles, counts.p, D, 1u);
-        }
+        // Rows go from the streaming kernel straight to their slabs.  Regrouping a whole tile by destination in shared
+        // memory first measured SLOWER at 2 ranks (6.64 vs 4.97 ms for 5*10^7 rows out): the 64-byte row stores already
+        // fill whole NVLink packets, staging only adds a shared-memory round trip and a barrier.
+        scatter_stream_kernel<<<(u32)tiles, kStreamThreads, 0, st>>>(reinterpret_cast<const uint4*>(in->rows), index.p, n, rb / 16, parts, bits,
+                                                                    tiles, counts.p, D);
         YTGPU_CUDA_TRY(cudaGetLastError());
     }
     {
